@@ -56,7 +56,15 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-sample-steps", type=int, default=40, help="env steps per episode in the CPU sample")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed generation computed as DIR/<name>.npy "
+                         "(es workload, b200 impl): the inputs are seeded, so two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "es"):
+        ap.error("--dump-outputs is implemented for --impl b200 --workload es")
+    return args
 
 
 def load_peaks():
@@ -183,8 +191,10 @@ def run_b200(args):
     for e in phase_ev:
         e.record()                                               # materialise the handles
     R = 4                                                        # observation pool blocks, rotated every tick
-    pool = torch.randint(0, 256, (R, slots, 84, 84, 4), dtype=torch.uint8, device=dev)
-    rew_pool = (torch.rand(64, slots, device=dev) < 0.05).float() * 10.0
+    gen = torch.Generator(device=dev)
+    gen.manual_seed(rank)                                        # same arguments -> same observations and rewards
+    pool = torch.randint(0, 256, (R, slots, 84, 84, 4), dtype=torch.uint8, device=dev, generator=gen)
+    rew_pool = (torch.rand(64, slots, device=dev, generator=gen) < 0.05).float() * 10.0
     ret_acc = torch.zeros(slots, device=dev)
     idx_stream = np.random.RandomState(1)
     tally = {"launches": 0, "pairs": 0}
@@ -223,6 +233,7 @@ def run_b200(args):
             bd.append((tag, time.perf_counter()))
 
     rollout_ev = []              # (start, end) CUDA events around the rollout part of every generation (this rank's own work)
+    last = {}                    # the latest generation's results (device tensors; read back only by --dump-outputs)
 
     def generation_value():
         mark("start")
@@ -238,6 +249,7 @@ def run_b200(args):
             npw = len(wave)
             per = -(-npw // NS)                                   # pairs per stream partition
             parts = [wave[h * per:(h + 1) * per] for h in range(NS)]
+            last["active_slots"] = [2 * len(p) for p in parts]
             for h in range(NS):
                 k = len(parts[h])
                 act = np.zeros(part, dtype=np.uint8)
@@ -310,6 +322,7 @@ def run_b200(args):
         g = upd.gradient(proc[lo:hi].contiguous(), torch.from_numpy(my).to(dev), denom=2 * n_pairs)
         shard.all_reduce_sum_(g)
         upd.step(L2)
+        last.update(returns=allret, centered_ranks=proc, gradient=g)
         mark("update")
         if BREAKDOWN:
             t0 = bd[0][1]
@@ -360,6 +373,15 @@ def run_b200(args):
         ms_val, clocks, launches, prof = timed(generation_value, args.steps, args.warmup, profile=True)
     finally:
         F.check(L.dne_set_option(b"chain_ticks", 0))
+    if args.dump_outputs and rank == 0:
+        # rank 0's results of the last timed generation: the updated parameters, the update's inputs, and the final tick's
+        # logits / actions on the slots the last wave used (before parity_check reuses the slot tables)
+        n_act = last["active_slots"]
+        dump_outputs(args.dump_outputs, {
+            "theta": upd.theta, "gradient": last["gradient"], "returns": last["returns"],
+            "centered_ranks": last["centered_ranks"],
+            "logits": torch.cat([sfs[h].logits[:n_act[h]] for h in range(NS)]),
+            "actions": torch.cat([sfs[h].actions[:n_act[h]] for h in range(NS)])})
     # this rank's own rollout time per generation (before the all_gather that synchronises the ranks): rank skew shows here
     my_roll = sum(a.elapsed_time(b) for a, b in rollout_ev[-args.steps:]) / args.steps
     roll_t = torch.tensor([my_roll], dtype=torch.float64, device=dev)
@@ -418,7 +440,7 @@ def run_b200(args):
         ES._STATE["ctx"] = ctx
         slots_e2e = -(-slots // 4) * 4                       # RolloutRunner: multiple of group (2) x pipeline halves (2)
         env = SyntheticAtariEnv(slots_e2e, episode_len=T, seed=rank)
-        marks = {}
+        marks = {0: time.perf_counter()}        # iterations count from 1: with --warmup 0 the window opens here
 
         io = {"h2d": 0, "d2h": 0}
 
@@ -471,6 +493,25 @@ def run_b200(args):
         _emit(line)
     if world > 1:
         dist.destroy_process_group()
+
+
+# ---------------------------------------------------------------------------------------------------------------
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, tensors):
+    """Write each tensor as out_dir/<name>.npy: float64 stays float64, everything else becomes float32 (integer actions are
+    exact in float32)."""
+    arrays = {}
+    for name, t in tensors.items():
+        a = t.detach().cpu().numpy()
+        arrays[name] = a if a.dtype == np.float64 else a.astype(np.float32)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ---------------------------------------------------------------------------------------------------------------

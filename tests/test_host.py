@@ -365,6 +365,17 @@ def test_bench_clock_sampler_and_reference_arm_contract(tmp_path):
     assert line["value"] > 0 and line["config"]["workload"].startswith("frostbite_es")
 
 
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--warmup", "-1"], ["--impl", "reference", "--dump-outputs", "d"],
+                                  ["--workload", "mlp", "--dump-outputs", "d"]])
+def test_bench_rejects_arguments_it_cannot_honour(argv, tmp_path):
+    """No timed step to report, or an output dump the chosen arm does not produce: an argument error, before any work."""
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py")] + argv, capture_output=True, text=True,
+                         timeout=120, cwd=tmp_path)
+    assert out.returncode == 2 and out.stdout == "", out.stderr[-2000:]
+    assert not os.path.exists(tmp_path / "d")
+
+
 def test_normc_initialiser_matches_reference_bit_exactly():
     """tf_util.normc_initializer (tf_util.py:108-119) executed by tests/golden/make_golden_policies.py on the global numpy stream
     vs the package's initialiser on a RandomState with the same seed."""
